@@ -15,6 +15,10 @@ N>1: inverted lists are packed onto the ranks by size; the SAME search call is a
 all-gather), bounds are min-reduced, every rank scans its own lists for the full batch, one all-gather of the
 per-shard top-k + merge kernel ("strong" scaling: fixed index and batch).  The N>1 line carries the proof that the
 merged result equals the unsharded one.  torch is plumbing here (device buffers, RNG, events, torch.distributed).
+
+--dump-outputs DIR writes what the last timed step returned (rank 0): DIR/ids.npy (float64, exact for int64 labels) and
+DIR/distances.npy (float32), nq x k each.  Inputs come from fixed seeds, so two builds run with the same arguments can be
+compared output for output.
 """
 import argparse
 import json
@@ -158,6 +162,12 @@ def recall_of(gt, ids):
     for a, b in zip(gt, ids):
         hit += len(set(a.tolist()) & set(b.tolist()) - {-1})
     return hit / float(gt.shape[0] * gt.shape[1])
+
+
+def dump_outputs(path, ids, dist):
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "ids.npy"), np.asarray(ids).astype(np.float64))
+    np.save(os.path.join(path, "distances.npy"), np.asarray(dist).astype(np.float32))
 
 
 def make_comm(kb, dist, rank, world, device_index):
@@ -330,6 +340,8 @@ def run_ours(args):
     if os.environ.get("KB2_PROFILE"):
         torch.cuda.cudart().cudaProfilerStop()
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, ids.cpu().numpy(), dis.cpu().numpy())
     ms_total = e0.elapsed_time(e1)
     if world > 1:
         t = torch.tensor([ms_total], device=dev)
@@ -578,9 +590,12 @@ def run_reference(args):
     for _ in range(args.warmup):
         r.search(xq_np, k, cfg["nprobe"], refine_k=rk, nthreads=nthreads)
     t0 = time.perf_counter()
+    I = D = None
     for _ in range(args.steps):
-        r.search(xq_np, k, cfg["nprobe"], refine_k=rk, nthreads=nthreads)
+        I, D = r.search(xq_np, k, cfg["nprobe"], refine_k=rk, nthreads=nthreads)
     el = time.perf_counter() - t0
+    if args.dump_outputs and I is not None:
+        dump_outputs(args.dump_outputs, I, D)
     qps = nq * args.steps / el
     out = {"impl": "reference", "metric": METRIC_NAME if args.workload == "ivf_pq_10m" else f"queries/sec, {args.workload}",
            "value": qps, "unit": "queries/s", "n_gpus": world, "steps": args.steps, "warmup": args.warmup,
@@ -609,6 +624,7 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="ivf_pq_10m", choices=sorted(WORKLOADS))
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's ids and distances to DIR/*.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":

@@ -30,13 +30,23 @@ def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a B200 (run with -m gpu on the GPU box)")
 
 
-@pytest.fixture(scope="session")
-def ref():
-    """compiled reference oracle (oracle/_ref); parity tests skip loudly if it did not travel"""
-    from oracle import ref as r
-    if not r.available():
-        pytest.skip("oracle/_ref/libknowhere_ref.so not built")
-    return r
+@pytest.fixture
+def ref(request):
+    """the compiled reference oracle's answers for this test, replayed from tests/golden/ref (oracle/tape.py);
+    KB2_RECORD_REF=1 records them from oracle/_ref instead"""
+    from oracle import tape
+    test_id = f"{request.node.module.__name__}::{request.node.name}"
+    session = tape.Recorder(test_id) if tape.recording() else tape.Player(test_id)
+    yield tape.Ref(session)
+    rep = getattr(request.node, "rep_call", None)
+    if tape.recording() and rep is not None and rep.passed:
+        session.save()
+
+
+@pytest.hookimpl(hookwrapper=True)
+def pytest_runtest_makereport(item, call):
+    rep = (yield).get_result()
+    setattr(item, "rep_" + rep.when, rep)
 
 
 @pytest.fixture(scope="session")

@@ -1,5 +1,5 @@
-"""Generates tests/golden/*.npz from the REFERENCE itself (oracle/_ref, compiled from /root/reference).
-Run here (where /root/reference exists):  python tests/golden/make_golden.py
+"""Generates tests/golden/*.npz from the REFERENCE itself (oracle/_ref, compiled by oracle/build_ref.py).
+Run where the reference sources exist:  python tests/golden/make_golden.py
 Inputs are regenerated from seeds by knowhere_b200.datagen; fixtures hold the reference's trained
 state and its answers, so the GPU box can check both the numpy oracle and the CUDA path without
 /root/reference."""
@@ -52,7 +52,12 @@ def ivf():
                 codes_all.append(codes.reshape(-1))
             out[f"{tag}_list_sizes"] = np.array(sizes, np.int64)
             out[f"{tag}_list_ids"] = np.concatenate(ids_all)
-            out[f"{tag}_list_codes"] = np.concatenate(codes_all)
+            codes_all = np.concatenate(codes_all)
+            if kind == "IVF_FLAT":
+                # IVF_FLAT codes are the base rows: the tests rebuild them from xb (keeps the fixture small)
+                assert np.array_equal(codes_all, xb[out[f"{tag}_list_ids"]].view(np.uint8).reshape(-1))
+            else:
+                out[f"{tag}_list_codes"] = codes_all
             I, D = r.search(xq, k, nprobe)
             out[f"{tag}_ids"], out[f"{tag}_dist"] = I, D
             CI, CD = r.coarse(xq, nprobe)

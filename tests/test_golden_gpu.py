@@ -29,7 +29,7 @@ def test_golden_ivf_gpu(kb, name, metric):
     nb, d, nq, k, nprobe, m = 4000, 64, 20, 10, 4, 8
     xb, xq = datagen.clustered(nb, d, 42), datagen.clustered(nq, d, 43)
     ix = kb.Index("IVF_FLAT", metric, d, {"nlist": 16})
-    L = _lists(z, "ivf_flat", d * 4)
+    L = _lists(z, "ivf_flat", d * 4, xb)
     ix.ivf_import(z["ivf_flat_centroids"], None, [(l,) + L[l] for l in sorted(L)])
     ids, dist = ix.search(xq, k, {"nprobe": nprobe})
     assert_topk_parity(ids, dist, z["ivf_flat_ids"], z["ivf_flat_dist"], what="golden IVF_FLAT")
